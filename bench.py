@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Lloyd-iteration samples/sec of the B200 KMeans engine (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1], "C2"): synthetic blobs 10M x 64 float32, k = 256, one chunk per GPU,
@@ -27,6 +27,12 @@ Numbers reported:
   cpu_baseline  the dask-ml path restated without dask (oracle/: scikit-learn float64 E-step + the reference's numba
                 scatter-add, thread pool over row blocks) on a bounded row sample of C2
 ``--impl reference`` times that CPU path alone on the FULL 10M-row C2 chunk and prints the same line shape.
+``--dump-outputs DIR`` writes what the last timed headline step computed (rank 0): ``centers.npy`` (k, d) float64,
+``labels.npy`` float32 (every row up to DUMP_LABEL_ROWS, else a fixed seeded sample of that many rows, in row order)
+and ``shift.npy`` (1,) float64.  The inputs depend only on the arguments, so two builds can be compared file by file,
+with a tolerance: the float64 re-check adds its deferred rows to the sums with atomics, so repeated runs differ in the
+last bits, and over many steps such a difference can flip a near-tied label and move the centres further (NVIDIA B200,
+1000 W limit, 20 steps: centres within 1e-7 in two of three repeats, within 3e-3 in the third).
 """
 import argparse
 import json
@@ -62,6 +68,8 @@ CONFIGS = {
                 what="slice of C5: 8M x 128 bf16 per GPU, k=1024 (C5 is 125M rows per GPU; samples/s is linear in n)"),
 }
 N_ROWS, N_FEAT, N_CLUST = CONFIGS["C2"]["n"], CONFIGS["C2"]["d"], CONFIGS["C2"]["k"]
+# --dump-outputs: at most 12M labels as float32 (48 MB), so that one dump stays under 64 MB
+DUMP_LABEL_ROWS = 12_000_000
 
 
 def _peaks():
@@ -333,17 +341,38 @@ def time_lloyd(st, steps, warmup, barrier, world, dev):
     barrier()
     l0 = st.be.launch_count()
     ev0.record()
-    lloyd_loop(st, steps, 0.0)
+    _, last, _ = lloyd_loop(st, steps, 0.0)
     ev1.record()
     barrier()
     launches = st.be.launch_count() - l0
     st.kernel_event_hook = None
+    if last + 1 != steps:
+        raise RuntimeError("the timed loop ran %d of %d iterations" % (last + 1, steps))
     ms_total = ev0.elapsed_time(ev1)
     kern_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
     t = torch.tensor([ms_total, kern_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     return float(t[0]) / steps, float(t[1]), int(launches)
+
+
+def dump_outputs(out_dir, st):
+    """Write what the last step of the timed loop computed (see the module docstring); returns the written shapes."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    labels = st.labels[0]
+    n = int(labels.shape[0])
+    if n > DUMP_LABEL_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LABEL_ROWS, replace=False))
+        labels = labels[torch.from_numpy(rows).to(labels.device)]
+    out = {"centers": st.C.cpu().numpy().astype(np.float64),
+           "labels": labels.cpu().numpy().astype(np.float32),
+           "shift": st.shift.cpu().numpy().astype(np.float64).reshape(1)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "label_rows": "%d of %d" % (out["labels"].shape[0], n),
+            "files": {name + ".npy": list(a.shape) for name, a in out.items()}}
 
 
 def _static_traffic(name):
@@ -438,7 +467,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer e2e leg")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3/C4/C5 sub-records")
     ap.add_argument("--configs", default="C3,C4,C5", help="comma-separated sub-records to run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the centres, labels and shift of the last timed headline step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -486,6 +519,7 @@ def main():
     clocks = sampler.stop()
     value = n * world / (ms_per_step * 1e-3)
     shift = float(st.shift.item())
+    dumped = dump_outputs(args.dump_outputs, st) if args.dump_outputs and rank == 0 else None
     C_used = st.C_new.clone()
     par = parity_check(X, st.labels[0], C_used, be, N_CLUST)
 
@@ -642,6 +676,8 @@ def main():
         "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline, "parity_check": par,
         "allreduce_us": allreduce_us, "transform": xform, "configs": configs, "cpu_baseline": cpu,
     }
+    if dumped:
+        line["dump_outputs"] = dumped
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

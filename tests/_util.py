@@ -1,5 +1,33 @@
 """Helpers shared by the parity tests."""
+import hashlib
+import os
+
 import numpy as np
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def blobs(n, d, k_true, seed, dtype):
+    """Isotropic blobs drawn from numpy's legacy ``RandomState``, whose streams numpy keeps fixed across releases:
+    the Lloyd fixtures in tests/golden/ store these parameters instead of the rows."""
+    rng = np.random.RandomState(seed)
+    cent = rng.uniform(-10, 10, size=(k_true, d))
+    return (cent[rng.randint(0, k_true, size=n)] + rng.standard_normal((n, d))).astype(dtype)
+
+
+def x_digest(X):
+    return hashlib.sha256(np.ascontiguousarray(X).tobytes()).hexdigest()
+
+
+def load_golden(name):
+    """A Lloyd fixture of tests/golden/ as a dict, with its input rows ``X`` regenerated from the stored
+    ``blobs`` parameters and checked against the SHA-256 of the rows the fixture was computed from."""
+    g = dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+    n, d, k_true, seed = (int(v) for v in g["blobs"])
+    X = blobs(n, d, k_true, seed, str(g["dtype"]))
+    assert x_digest(X) == str(g["X_sha256"]), "%s: regenerated input rows differ from the fixture's" % name
+    g["X"] = X
+    return g
 
 
 def d2_f64(X, C):

@@ -6,7 +6,9 @@ The reference (mrocklin/dask-ml) cannot be imported in the build image (dask is 
 are produced by the oracle restatement (oracle/kmeans_oracle.py), whose per-chunk arithmetic is the
 reference's own dependency (scikit-learn pairwise_distances_argmin_min) plus the restated scatter-add,
 and whose results are asserted equal to scikit-learn's Lloyd in tests/test_oracle.py exactly as the
-reference's tests do.  scikit-learn / numpy versions are recorded in MANIFEST.json.
+reference's tests do.  scikit-learn / numpy versions are recorded in MANIFEST.json.  The input rows are not
+stored: a fixture keeps the parameters of ``tests/_util.blobs`` and the SHA-256 of the rows it was computed from
+(``tests/_util.load_golden`` regenerates and checks them).
 """
 import json
 import os
@@ -16,14 +18,9 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+sys.path.insert(0, os.path.dirname(HERE))
 from oracle import kmeans_oracle as ok  # noqa: E402
-
-
-def blobs(n, d, k_true, seed, dtype):
-    rng = np.random.RandomState(seed)
-    cent = rng.uniform(-10, 10, size=(k_true, d))
-    return (cent[rng.randint(0, k_true, size=n)] + rng.standard_normal((n, d))).astype(dtype)
-
+from _util import blobs, x_digest  # noqa: E402
 
 CASES = {
     # name: (n, d, k, k_true, dtype, chunks, max_iter, tol, seed)
@@ -41,7 +38,8 @@ def main():
         init = X[:k].copy()
         lab, inertia, C, n_iter = ok.kmeans_single_lloyd(ok.to_blocks(X, chunks), k, init=init, max_iter=max_iter,
                                                         tol=tol)
-        np.savez_compressed(os.path.join(HERE, name + ".npz"), X=X, init=init, k=k, chunks=chunks,
+        np.savez_compressed(os.path.join(HERE, name + ".npz"), blobs=np.array([n, d, kt, seed]), dtype=dt,
+                            X_sha256=x_digest(X), init=init, k=k, chunks=chunks,
                             max_iter=max_iter, tol=tol, labels=np.concatenate(lab), centers=C,
                             inertia=inertia, n_iter=n_iter)
         manifest["cases"][name] = {"n": n, "d": d, "k": k, "dtype": dt, "n_iter": int(n_iter),

@@ -14,8 +14,9 @@ therefore runs through the reference's own code: its graph construction (``pairw
 ``_centers_dense`` and its Lloyd control flow.
 
 The outputs are written as golden fixtures (inputs + reference outputs) that tests/test_oracle.py replays
-against the oracle and tests/test_gpu_kmeans.py against the CUDA engine on the GPU box, where /root/reference
-does not exist.
+against the oracle and tests/test_gpu_kmeans.py against the CUDA engine, without the reference checkout.  The
+Lloyd fixtures store the parameters of ``tests/_util.blobs`` and the SHA-256 of the input rows instead of the
+rows themselves (``tests/_util.load_golden`` regenerates and checks them).
 """
 import collections
 import collections.abc
@@ -28,6 +29,8 @@ import numpy as np
 
 REF = os.environ.get("BKM_REFERENCE", "/root/reference")
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE))
+from _util import blobs, x_digest  # noqa: E402
 
 
 # --------------------------------------------------------------------------------------------------
@@ -328,12 +331,6 @@ def install():
 # --------------------------------------------------------------------------------------------------
 # fixture generation
 # --------------------------------------------------------------------------------------------------
-def _blobs(n, d, k_true, seed, dtype):
-    rng = np.random.RandomState(seed)
-    cent = rng.uniform(-10, 10, size=(k_true, d))
-    return (cent[rng.randint(0, k_true, size=n)] + rng.standard_normal((n, d))).astype(dtype)
-
-
 CASES = {
     # name: (n, d, k, k_true, dtype, chunks, max_iter, tol, seed)
     "ref_lloyd_f32_64x256": (6000, 64, 256, 80, "float32", 2500, 6, 1e-4, 21),
@@ -348,20 +345,21 @@ def main():
     da, KM = ref.da, ref.k_means.KMeans
     manifest = {}
     for name, (n, d, k, kt, dt, chunks, max_iter, tol, seed) in CASES.items():
-        X = _blobs(n, d, kt, seed, dt)
+        X = blobs(n, d, kt, seed, dt)
         init = X[:k].copy()
         Xd = da.from_array(X, chunks=(chunks, d))
         est = KM(n_clusters=k, init=init, max_iter=max_iter, tol=tol).fit(Xd)          # the reference's own fit
         labels = np.asarray(est.labels_.compute())
         pred = np.asarray(est.predict(Xd).compute())
         trans = np.asarray(est.transform(Xd).compute())
-        np.savez_compressed(os.path.join(HERE, name + ".npz"), X=X, init=init, k=k, chunks=chunks, max_iter=max_iter,
+        np.savez_compressed(os.path.join(HERE, name + ".npz"), blobs=np.array([n, d, kt, seed]), dtype=dt,
+                            X_sha256=x_digest(X), init=init, k=k, chunks=chunks, max_iter=max_iter,
                             tol=tol, labels=labels, centers=est.cluster_centers_, inertia=np.float64(est.inertia_),
                             n_iter=est.n_iter_, predict=pred, transform=trans[:256])
         manifest[name] = dict(n=n, d=d, k=k, dtype=dt, n_iter=int(est.n_iter_), inertia=float(est.inertia_))
         print(name, manifest[name])
     # per-chunk operator pins (reference tests/metrics/test_metrics.py:16-43)
-    Xc = _blobs(1000, 4, 5, 31, "float64")
+    Xc = blobs(1000, 4, 5, 31, "float64")
     centers = Xc[::100]
     a, b = ref.pairwise.pairwise_distances_argmin_min(da.from_array(Xc, chunks=(500, 4)), centers)
     pd_ = ref.pairwise.pairwise_distances(da.from_array(Xc, chunks=(500, 4)), centers)

@@ -5,7 +5,7 @@ import pytest
 import sklearn.datasets
 from sklearn.cluster import KMeans as SKKMeans, kmeans_plusplus
 
-from _util import assert_labels_match
+from _util import assert_labels_match, load_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -229,12 +229,10 @@ REF_CASES = ["ref_lloyd_f32_64x256", "ref_lloyd_f64_16x8", "ref_lloyd_f32_41x100
 def test_engine_matches_fixtures_written_by_the_reference(name):
     """The CUDA engine against outputs of the UNMODIFIED reference code (tests/golden/ref_shim.py): same
     n_iter, labels (modulo float64 near-ties), centres, inertia (both Q4 branches), predict and transform."""
-    import os
-
     from dask_ml_b200 import ChunkedArray
     from dask_ml_b200.cluster import KMeans
 
-    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name + ".npz"))
+    g = load_golden(name)
     X = ChunkedArray.from_array(g["X"], int(g["chunks"]))
     km = KMeans(int(g["k"]), init=g["init"], max_iter=int(g["max_iter"]), tol=float(g["tol"])).fit(X)
     assert km.n_iter_ == int(g["n_iter"])

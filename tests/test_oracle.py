@@ -11,6 +11,8 @@ import sklearn.metrics
 from sklearn.cluster import KMeans as SKKMeans, kmeans_plusplus
 from sklearn.utils.extmath import row_norms
 
+from _util import load_golden
+
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
@@ -145,8 +147,7 @@ def test_philox_known_answers(oracle):
 def test_golden_fixtures(oracle, name):
     """Committed golden vectors (tests/golden/make_golden.py): the oracle must reproduce them bit for bit
     on labels and to 1e-12 on centres/inertia (guards the oracle against dependency drift)."""
-    path = os.path.join(GOLD, name + ".npz")
-    g = np.load(path)
+    g = load_golden(name)
     blocks = oracle.to_blocks(g["X"], int(g["chunks"]))
     lab, inertia, C, n_iter = oracle.kmeans_single_lloyd(blocks, int(g["k"]), init=g["init"],
                                                         max_iter=int(g["max_iter"]), tol=float(g["tol"]))
@@ -165,7 +166,7 @@ def test_oracle_reproduces_the_reference_itself(oracle, name):
     (dask_ml/cluster/k_means.py, metrics/pairwise.py, utils.py) executed over an eager stand-in for dask:
     KMeans(init=ndarray).fit -> labels_, cluster_centers_, inertia_, n_iter_.  The oracle must agree bit for bit
     on labels / n_iter and to float64 round-off on centres and inertia (both inertia branches of Q4 occur)."""
-    g = np.load(os.path.join(GOLD, name + ".npz"))
+    g = load_golden(name)
     blocks = oracle.to_blocks(g["X"], int(g["chunks"]))
     lab, inertia, C, n_iter = oracle.kmeans_single_lloyd(blocks, int(g["k"]), init=g["init"],
                                                         max_iter=int(g["max_iter"]), tol=float(g["tol"]))
